@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- queries/sec top-10 over the synthetic PQ96 phrase index (BASELINE.json metric), one process per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path
   python bench.py --impl reference [...]                          # the reference's CPU path (FAISS-equivalent restatement)
 
 A *step* is one pass of the hot path (OPQ rotation -> coarse top-nprobe -> LUT -> PQ96 scan -> top-k merge) over one
@@ -532,6 +532,8 @@ def run_ours(args):
     Q, Qh = queries(ix, wl, W + K)
     stage(f"{wl['name']} index built ({ix.local.device_bytes / 1e9:.1f} GB on this rank), queries made")
     main = measure_search(cx, ix, wl, Q, Qh, wl["nprobe"], sample_clocks=True)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, *main["_last"])
     second = None
     if wl["name"] == "C4":
         second = measure_search(cx, ix, wl, Q, Qh, 32)
@@ -590,6 +592,14 @@ def run_ours(args):
     return 0
 
 
+def dump_outputs(out_dir, D, I):
+    """What the last timed step of the headline search returned to its caller: top-k scores (fp32) and labels (int64, stored as
+    float64, exact below 2^53), each [batch, k].  The queries are seeded, so two builds run with the same arguments can be compared."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scores.npy"), np.asarray(D, dtype=np.float32))
+    np.save(os.path.join(out_dir, "labels.npy"), np.asarray(I).astype(np.float64))
+
+
 def c1_leg(cx, build, queries, args):
     """C1 (BASELINE.json configs[0]): IVF1,PQ96, 1M phrases, 100 queries -- the reference's own CPU-runnable case, on the GPU and
     through the CPU oracle on the same 100 queries."""
@@ -631,25 +641,20 @@ def c4_single_gpu_leg(cx, build, queries, args):
     """C4's index (1B phrases, IVF65536, 96 GB of codes) held by ONE B200, batch 1024: the N = 1 point of the metric's 1/2/4/8 series."""
     import torch
     wl = workload("C4", args.scale)
-    save = (cx.W, cx.K)
-    cx.W, cx.K = 3, max(5, min(cx.K, 20))
-    try:
-        ix = build(wl)
-        Q, Qh = queries(ix, wl, cx.W + cx.K)
-        out = {"steps": cx.K, "warmup": cx.W}
-        for nprobe in (wl["nprobe"], 32):
-            m = measure_search(cx, ix, wl, Q, Qh, nprobe)
-            r = {k_: v for k_, v in m.items() if not k_.startswith("_") and k_ != "clocks"}
-            r["config"] = config_dict(wl, 1, nprobe)
-            if not args.no_cpu:
-                oc = oracle_check(cx, wl, nprobe, Qh[cx.W + cx.K - 1], m["_last"], 16)
-                r["oracle_check"] = {k_: oc[k_] for k_ in OC_KEYS}
-            out[f"nprobe{nprobe}"] = r
-        del ix
-        torch.cuda.empty_cache()
-        return out
-    finally:
-        cx.W, cx.K = save
+    ix = build(wl)
+    Q, Qh = queries(ix, wl, cx.W + cx.K)
+    out = {"steps": cx.K, "warmup": cx.W}
+    for nprobe in (wl["nprobe"], 32):
+        m = measure_search(cx, ix, wl, Q, Qh, nprobe)
+        r = {k_: v for k_, v in m.items() if not k_.startswith("_") and k_ != "clocks"}
+        r["config"] = config_dict(wl, 1, nprobe)
+        if not args.no_cpu:
+            oc = oracle_check(cx, wl, nprobe, Qh[cx.W + cx.K - 1], m["_last"], 16)
+            r["oracle_check"] = {k_: oc[k_] for k_ in OC_KEYS}
+        out[f"nprobe{nprobe}"] = r
+    del ix
+    torch.cuda.empty_cache()
+    return out
 
 
 def encoder_leg(cx, ix, wl):
@@ -778,10 +783,16 @@ def main():
     ap.add_argument("--no-encoder", action="store_true", help="skip the C3 encoder leg")
     ap.add_argument("--no-c1", action="store_true", help="skip the C1 leg")
     ap.add_argument("--no-c4", action="store_true", help="N=1: skip the C4-on-one-GPU leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the top-k scores and labels of the last timed step of the headline search to DIR/{scores,labels}.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.steps is None:
         args.steps = 10 if args.impl == "reference" else 100
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records this repo's CUDA path (--impl ours)")
     quiet_stdout()
     return run_reference(args) if args.impl == "reference" else run_ours(args)
 

@@ -2,6 +2,8 @@
 lists), queries, and the oracle's outputs (C restatement, cross-checked against the numpy restatement and the fp64
 brute force before writing).  The reference repo has no golden vectors for this path (SURVEY.md 8c) and faiss cannot be
 installed here, so these pin the *restatement* (and through it the CUDA path) against silent drift.
+The matrix, codebooks, centroids and codes come from the oracle's seeded integer-hash generators, which give the same bits on
+every platform, so only labels, queries and outputs are stored (tests.helpers.load_ivfpq_small rebuilds the rest).
 Run from the repo root:  python tests/golden/make_golden.py"""
 import json
 import os
@@ -12,20 +14,22 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import ivfpq_ref as R  # noqa: E402
+from tests.helpers import ivfpq_small_arrays  # noqa: E402
 
 if __name__ == "__main__":
     R.build()
-    seed, nlist, k, nprobe = 777, 24, 10, 6
+    # opq_seed / opq_sigma: a dense seeded matrix stands in for the OPQ rotation (the search does not assume orthogonality)
+    meta = {"seed": 777, "opq_seed": 778, "opq_sigma": 0.036, "k": 10, "nprobe": 6, "generator": "tests/golden/make_golden.py",
+            "oracle": "oracle/ivfpq_ref.c"}
+    seed, nlist, k, nprobe = meta["seed"], 24, meta["k"], meta["nprobe"]
     rng = np.random.default_rng(seed)
     lens = rng.integers(0, 90, nlist).astype(np.int64)
     lens[[2, 23]] = 0
     lens[5] = 33
-    A = np.linalg.qr(rng.standard_normal((768, 768)))[0].astype(np.float32)
-    pq = R.gen_pq(seed)
-    Cm = R.gen_centroids(seed, 0, nlist)
-    codes = np.concatenate([R.gen_codes(seed, l, 0, int(lens[l])) for l in range(nlist)])
+    g = ivfpq_small_arrays(R, meta, lens)
+    A = g["A"]
     ids = (rng.permutation(int(lens.sum())) * 5 + 3).astype(np.int64)
-    ix = R.RefIndex(A, pq, lens, centroids=Cm, codes=codes, ids=ids)
+    ix = R.RefIndex(A, g["pq"], lens, centroids=g["centroids"], codes=g["codes"], ids=ids)
     pick = rng.integers(0, len(ids), 12)
     x = (ix.reconstruct(ids[pick])[0] @ A + 0.3 * rng.standard_normal((12, 768))).astype(np.float32)
     D, I, key = ix.search(x, k, nprobe, return_key=True)
@@ -34,8 +38,6 @@ if __name__ == "__main__":
     Db, Ib = R.brute_force_fp64(ix, x, key, k)
     assert np.abs(Db - D).max() < 1e-3 and (Ib == I).mean() > 0.97   # 1e-3 = the north-star score tolerance
     out = os.path.dirname(os.path.abspath(__file__))
-    np.savez_compressed(os.path.join(out, "ivfpq_small.npz"), A=A.astype(np.float16).astype(np.float32) if False else A, pq=pq, centroids=Cm,
-                        list_len=lens, codes=codes, ids=ids, x=x, D=D, I=I, key=key, recon0=ix.reconstruct(I[0])[0])
-    json.dump({"seed": seed, "k": k, "nprobe": nprobe, "generator": "tests/golden/make_golden.py", "oracle": "oracle/ivfpq_ref.c"},
-              open(os.path.join(out, "ivfpq_small.json"), "w"))
+    np.savez_compressed(os.path.join(out, "ivfpq_small.npz"), list_len=lens, ids=ids, x=x, D=D, I=I, key=key, recon0=ix.reconstruct(I[0])[0])
+    json.dump(meta, open(os.path.join(out, "ivfpq_small.json"), "w"))
     print("wrote", out)

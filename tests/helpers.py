@@ -23,6 +23,36 @@ def near_queries(ref, n, seed, noise=0.3):
     return (q + noise * rng.standard_normal(q.shape)).astype(np.float32)
 
 
+def ivfpq_small_arrays(oracle, meta, list_len):
+    """The seeded part of the tests/golden/ivfpq_small index: matrix, PQ codebooks, centroids and codes from the oracle's generators."""
+    seed, nlist = meta["seed"], len(list_len)
+    return {"A": oracle.gen_centroids(meta["opq_seed"], 0, D_MODEL, D_MODEL, meta["opq_sigma"]), "pq": oracle.gen_pq(seed),
+            "centroids": oracle.gen_centroids(seed, 0, nlist),
+            "codes": np.concatenate([oracle.gen_codes(seed, l, 0, int(list_len[l])) for l in range(nlist)])}
+
+
+def load_ivfpq_small(oracle):
+    """tests/golden/ivfpq_small.{npz,json} (tests/golden/make_golden.py) as (arrays, meta), the seeded arrays regenerated."""
+    import json
+    import os
+    gd = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    meta = json.load(open(os.path.join(gd, "ivfpq_small.json")))
+    g = dict(np.load(os.path.join(gd, "ivfpq_small.npz")))
+    g.update(ivfpq_small_arrays(oracle, meta, g["list_len"]))
+    return g, meta
+
+
+def jsonable(obj):
+    """`obj` as it reads back from a JSON golden file: tuples become lists, numpy scalars and arrays Python values."""
+    import json
+
+    def numpy_value(o):
+        if isinstance(o, (np.ndarray, np.generic)):
+            return o.tolist()
+        raise TypeError(f"not JSON serializable: {type(o).__name__}")
+    return json.loads(json.dumps(obj, default=numpy_value))
+
+
 def assert_topk_equal(D, I, Dref, Iref, what=""):
     """Bit-identical scores; identical labels up to permutations inside exactly-equal-score groups (faiss' heap
     order among equal scores is unspecified); in the boundary group only the group size is compared."""

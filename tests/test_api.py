@@ -6,16 +6,128 @@ import os
 import numpy as np
 import pytest
 
+from tests.helpers import jsonable
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def reference_golden(section):
+    """What the unmodified reference code returned on the inputs defined in this module (tests/golden/reference_api.json,
+    written by tests/golden/make_reference_api_golden.py)."""
+    return json.load(open(os.path.join(GOLD, "reference_api.json")))[section]
+
+
+# ---- inputs shared by the tests below and by tests/golden/make_reference_api_golden.py -----------------------------------------
+EVAL_QA = [("which river crosses the city", ["the Seine", "Seine"]), ("who signed the treaty", ["Louis XIV"]), ("what year", ["1648", "in 1648"]),
+           ("where", ["Paris"]), ("what is the a an the", ["yes"])]
+EVAL_CANNED = {"which river crosses the city": ["Seine", "Loire"], "who signed the treaty": ["Louis XV", "Louis XIV", "x"], "what year": [],
+               "where": ["paris.", "Lyon"], "what is the a an the": ["no", "Yes!"]}
+SEARCH_UNITS = ["phrase", "sentence", "paragraph", "document"]
+SEARCH_QUESTIONS = ["first question", "second question", "third"]
+QA_PAIRS_DATA = {"data": [{"id": "a1", "question": "Which river?", "answers": ["Seine"]},
+                          {"id": "a2", "origin": "nq.dev.x", "question": "who signed it", "answers": ["Louis", "Anne"], "titles": ["T1", "T2"]},
+                          {"id": "a3", "question": "skipped", "answers": []},
+                          {"id": "a4", "question": "x" * 400 + " [START_ENT] Paris [END_ENT] " + "y" * 400 + "?", "answers": ["Paris"]},
+                          {"id": "a5", "question": "ALL CAPS?", "answers": ["x"]}]}
+QA_PAIRS_CONFIGS = [(False, None), (True, None), (False, 1), (False, 3)]          # (do_lower_case, q_idx)
+BACKWARD_COMPAT_SD = {"bert_q_start.embeddings.w": 1, "bert_q_end.x": 2, "bert_start.y": 3, "cross_encoder.z": 4, "bert_qd.q": 5, "qa_outputs.w": 6,
+                      "query_start_encoder.k": 7, "linear.weight": 8}
+OPTION_GROUPS = ("add_model_options", "add_index_options", "add_retrieval_options", "add_data_options")
+OPTION_ARGV = ["--cuda", "--top_k", "40", "--nprobe", "64", "--index_name", "start/1048576_flat_OPQ96", "--eval_batch_size", "32", "--agg_strat", "opt2"]
+
+
+def eval_setup(tmp_path):
+    """Question file, parsed options and CPU stand-ins (encoder, phrase index with canned answers) for the evaluate loop."""
+    import torch
+    from densephrases import Options
+    from densephrases_b200.tokenization import WordPieceTokenizer
+    json.dump({"data": [{"id": str(i), "question": q, "answers": a} for i, (q, a) in enumerate(EVAL_QA)]}, open(os.path.join(tmp_path, "test.json"), "w"))
+    o = Options()
+    o.add_model_options(); o.add_index_options(); o.add_retrieval_options(); o.add_data_options()
+    args = o.parse(["--test_path", os.path.join(tmp_path, "test.json"), "--load_dir", str(tmp_path), "--top_k", "3", "--eval_batch_size", "2", "--save_pred"])
+
+    class FakeEncoder:
+        def __call__(self, input_ids_=None, attention_mask_=None, token_type_ids_=None, return_query=False):
+            assert return_query and input_ids_.shape == attention_mask_.shape == token_type_ids_.shape and input_ids_.shape[1] == args.max_query_length
+            b = input_ids_.shape[0]
+            return torch.ones((b, 1, 768)), torch.zeros((b, 1, 768))
+
+        def eval(self):
+            return self
+
+    class FakeMips:
+        num_docs_list = [1.0]
+
+        def search(self, query, q_texts=None, nprobe=256, top_k=10, max_answer_length=10, aggregate=False, agg_strat='opt1', return_sent=False):
+            assert query.shape == (len(q_texts), 1536) and top_k == 3
+            return [[{"answer": a, "context": "ctx " + a, "title": ["T"], "score": 10.0 - j, "start_pos": 4, "end_pos": 4 + len(a)}
+                     for j, a in enumerate(EVAL_CANNED[q])] for q in q_texts]
+
+    return args, FakeMips(), FakeEncoder(), WordPieceTokenizer.from_pretrained_or_synthetic(None)
+
+
+def search_setup(oracle):
+    """(query2vec, MIPS over the CPU oracle index, parsed options) that DensePhrases.search runs on."""
+    import torch
+    from densephrases import Options
+    from densephrases_b200 import runtime as R
+    from densephrases_b200.mips import MIPS
+    from densephrases_b200.tokenization import WordPieceTokenizer
+    from tests.test_mips import OracleIndexAdapter, build
+    doc_groups, idx_f, _, ref, query = build(oracle)
+    mips = MIPS.from_components(OracleIndexAdapter(ref), idx_f, doc_groups, cuda=False)
+    qvec = torch.from_numpy(query.astype(np.float32))
+
+    class FakeEncoder:
+        def __call__(self, input_ids_=None, attention_mask_=None, token_type_ids_=None, return_query=False):
+            b = input_ids_.shape[0]
+            return qvec[:b, None, :768], qvec[:b, None, 768:]
+
+    o = Options()
+    o.add_model_options(); o.add_index_options(); o.add_retrieval_options(); o.add_data_options()
+    args = o.parse([])
+    q2v = R.get_query2vec(query_encoder=FakeEncoder(), tokenizer=WordPieceTokenizer.from_pretrained_or_synthetic(None), args=args, batch_size=64)
+    return q2v, mips, args
+
+
+def search_outputs(model, unit):
+    """DensePhrases.search results compared across implementations: batch answers, metadata without the vectors, one single query."""
+    a = model.search(SEARCH_QUESTIONS, retrieval_unit=unit, top_k=3, truecase=False, return_meta=True)
+    strip = [[{k: v for k, v in r.items() if k not in ("start_vec", "end_vec")} for r in ret] for ret in a[1]]
+    single = model.search(SEARCH_QUESTIONS[0], retrieval_unit=unit, top_k=2, truecase=False)
+    return jsonable({"answers": a[0], "meta": strip, "single": single})
+
+
+class QaPairsArgs:
+    do_lower_case, draft, truecase, truecase_path = False, False, False, ""
+
+
+def truecase_differential_inputs(tables):
+    """Random sentences (x 3 out-of-vocabulary policies) and score queries over the vocabulary of tests/golden/truecase.dist."""
+    import random
+    rng = random.Random(12345)
+    vocab = list(tables["word_casing_lookup"]) + ["zzz", "o'brien", "42", "?", ",", "'s", "x-ray", "Ünïcode", "a.b"]
+    cases = []
+    for _ in range(400):
+        s = " ".join(rng.choice(vocab) for _ in range(rng.randint(0, 12)))
+        s = rng.choice([s, s.upper(), s.title(), "  " + s + " "])
+        cases += [(s, oov) for oov in ("title", "lower", "as-is")]
+    multi = [w for w, c in tables["word_casing_lookup"].items() if len(c) > 1]
+    scores = []
+    for _ in range(300):
+        tok = rng.choice(tables["word_casing_lookup"][rng.choice(multi)])
+        scores.append((rng.choice([None] + vocab), tok, rng.choice([None] + vocab)))
+    return cases, scores
+
 
 def test_reference_eval_script_imports_against_facade():
-    ref = "/root/reference/eval_phrase_retrieval.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present (GPU box)")
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_eval_phrase_retrieval", ref)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)                       # executes its `import faiss`, `from densephrases... import ...` lines (:12,:19-25)
-    assert callable(mod.evaluate) and callable(mod.embed_all_query)
+    """Every `densephrases...` / `faiss` import of the reference's eval_phrase_retrieval.py (recorded in the golden file) resolves
+    against this repo's facade; the `faiss` stub imports but refuses to be used."""
+    import importlib
+    for imp in reference_golden("eval_script_imports"):
+        mod = importlib.import_module(imp["module"])
+        for name in imp["names"]:
+            assert hasattr(mod, name), (imp["module"], name)
     import faiss
     with pytest.raises(RuntimeError):
         faiss.read_index
@@ -160,170 +272,69 @@ def test_metrics_match_reference_golden():
 def test_unmodified_reference_evaluate_runs_on_the_facade(tmp_path):
     """The reference's own `eval_phrase_retrieval.evaluate` (:49-91) + `evaluate_results` (:94-204), UNMODIFIED, executed over this
     repo's drop-in surface: `Options`, `load_qa_pairs`, `get_query2vec` (+ tokenizer) and the metric functions come from the
-    `densephrases` facade; only the phrase index and the encoder are CPU stand-ins with the documented call signatures.  Its
-    numbers equal densephrases_b200.runtime.evaluate on the same inputs (the reference reports percentages)."""
-    ref = "/root/reference/eval_phrase_retrieval.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present (GPU box)")
-    import importlib.util
-    import torch
-    from densephrases import Options
+    `densephrases` facade; only the phrase index and the encoder are CPU stand-ins with the documented call signatures (eval_setup).
+    What it returned and the prediction file it wrote are recorded in the golden file; densephrases_b200.runtime.evaluate gives the
+    same numbers (the reference reports percentages), predictions and scores on the same inputs."""
     from densephrases_b200 import runtime as R
-    from densephrases_b200.tokenization import WordPieceTokenizer
-    spec = importlib.util.spec_from_file_location("ref_eval_phrase_retrieval_run", ref)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    qa = [("which river crosses the city", ["the Seine", "Seine"]), ("who signed the treaty", ["Louis XIV"]), ("what year", ["1648", "in 1648"]),
-          ("where", ["Paris"]), ("what is the a an the", ["yes"])]
-    json.dump({"data": [{"id": str(i), "question": q, "answers": a} for i, (q, a) in enumerate(qa)]}, open(tmp_path / "test.json", "w"))
-    o = Options()
-    o.add_model_options(); o.add_index_options(); o.add_retrieval_options(); o.add_data_options()
-    args = o.parse(["--test_path", str(tmp_path / "test.json"), "--load_dir", str(tmp_path), "--top_k", "3", "--eval_batch_size", "2", "--save_pred"])
-    canned = {"which river crosses the city": ["Seine", "Loire"], "who signed the treaty": ["Louis XV", "Louis XIV", "x"], "what year": [],
-              "where": ["paris.", "Lyon"], "what is the a an the": ["no", "Yes!"]}
-
-    class FakeEncoder:
-        def __call__(self, input_ids_=None, attention_mask_=None, token_type_ids_=None, return_query=False):
-            assert return_query and input_ids_.shape == attention_mask_.shape == token_type_ids_.shape and input_ids_.shape[1] == args.max_query_length
-            b = input_ids_.shape[0]
-            return torch.ones((b, 1, 768)), torch.zeros((b, 1, 768))
-
-        def eval(self):
-            return self
-
-    class FakeMips:
-        num_docs_list = [1.0]
-
-        def search(self, query, q_texts=None, nprobe=256, top_k=10, max_answer_length=10, aggregate=False, agg_strat='opt1', return_sent=False):
-            assert query.shape == (len(q_texts), 1536) and top_k == 3
-            return [[{"answer": a, "context": "ctx " + a, "title": ["T"], "score": 10.0 - j, "start_pos": 4, "end_pos": 4 + len(a)}
-                     for j, a in enumerate(canned[q])] for q in q_texts]
-
-    tok = WordPieceTokenizer.from_pretrained_or_synthetic(None)
-    em1, f11, emk, f1k = mod.evaluate(args, mips=FakeMips(), query_encoder=FakeEncoder(), tokenizer=tok)
-    mine = R.evaluate(args, mips=FakeMips(), query_encoder=FakeEncoder(), tokenizer=tok)
-    assert (em1, f11, emk, f1k) == pytest.approx((100 * mine["exact_match_top1"], 100 * mine["f1_score_top1"], 100 * mine["exact_match_top3"],
-                                                  100 * mine["f1_score_top3"]))
-    assert em1 == pytest.approx(40.0) and emk == pytest.approx(80.0)
-    pred = json.load(open(tmp_path / "pred" / "test_5_top3.pred"))                       # written by the reference (:187-196)
-    assert pred["1"]["prediction"] == canned["who signed the treaty"] and pred["2"]["prediction"] == [""]
+    g = reference_golden("evaluate")
+    args, mips, enc, tok = eval_setup(tmp_path)
+    mine = R.evaluate(args, mips=mips, query_encoder=enc, tokenizer=tok)
+    assert (g["em1"], g["f11"], g["emk"], g["f1k"]) == pytest.approx((100 * mine["exact_match_top1"], 100 * mine["f1_score_top1"],
+                                                                      100 * mine["exact_match_top3"], 100 * mine["f1_score_top3"]))
+    assert g["em1"] == pytest.approx(40.0) and g["emk"] == pytest.approx(80.0)
+    pred = g["pred"]                                                                     # written by the reference (:187-196)
+    assert pred["1"]["prediction"] == EVAL_CANNED["who signed the treaty"] and pred["2"]["prediction"] == [""]
+    assert mine["predictions"] == [pred[str(i)]["prediction"] for i in range(len(EVAL_QA))]
+    assert mine["scores"] == [pred[str(i)]["score"] for i in range(len(EVAL_QA))]
 
 
-@pytest.mark.parametrize("unit", ["phrase", "sentence", "paragraph", "document"])
+@pytest.mark.parametrize("unit", SEARCH_UNITS)
 def test_densephrases_search_wrapper_equals_unmodified_reference_class(oracle, unit):
     """model.py:55-109 (`DensePhrases.search`: query2vec -> stacked vectors -> MIPS.search with the unit's aggregation -> field
-    selection) run UNMODIFIED over this repo's MIPS / query2vec gives exactly what densephrases_b200's DensePhrases.search returns."""
-    ref_path = "/root/reference/densephrases/model.py"
-    if not os.path.exists(ref_path):
-        pytest.skip("reference tree not present (GPU box)")
-    import importlib.util
-    import sys
-    import types
-    import torch
-    from densephrases import DensePhrases, Options
-    from densephrases_b200 import runtime as R
-    from densephrases_b200.mips import MIPS
-    from densephrases_b200.tokenization import WordPieceTokenizer
-    from tests.test_mips import OracleIndexAdapter, build
-    stub = types.ModuleType("densephrases.utils.squad_utils")
-    stub.TrueCaser = type("TrueCaser", (), {})
-    sys.modules["densephrases.utils.squad_utils"] = stub
-    try:
-        spec = importlib.util.spec_from_file_location("ref_densephrases_model", ref_path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-    finally:
-        del sys.modules["densephrases.utils.squad_utils"]
-    doc_groups, idx_f, _, ref, query = build(oracle)
-    mips = MIPS.from_components(OracleIndexAdapter(ref), idx_f, doc_groups, cuda=False)
-    qvec = torch.from_numpy(query.astype(np.float32))
-
-    class FakeEncoder:
-        def __call__(self, input_ids_=None, attention_mask_=None, token_type_ids_=None, return_query=False):
-            b = input_ids_.shape[0]
-            return qvec[:b, None, :768], qvec[:b, None, 768:]
-
-    o = Options()
-    o.add_model_options(); o.add_index_options(); o.add_retrieval_options(); o.add_data_options()
-    args = o.parse([])
-    q2v = R.get_query2vec(query_encoder=FakeEncoder(), tokenizer=WordPieceTokenizer.from_pretrained_or_synthetic(None), args=args, batch_size=64)
-    theirs, ours = mod.DensePhrases.__new__(mod.DensePhrases), DensePhrases.__new__(DensePhrases)
-    for obj in (theirs, ours):
-        obj.query2vec, obj.mips, obj.truecase, obj.args = q2v, mips, None, args
-    qs = ["first question", "second question", "third"]
-    a = theirs.search(qs, retrieval_unit=unit, top_k=3, truecase=False, return_meta=True)
-    b = ours.search(qs, retrieval_unit=unit, top_k=3, truecase=False, return_meta=True)
-    assert a[0] == b[0] and len(a[0]) == 3 and all(len(x) <= 3 for x in a[0])
-    strip = lambda rets: [[{k: v for k, v in r.items() if k not in ("start_vec", "end_vec")} for r in ret] for ret in rets]
-    assert strip(a[1]) == strip(b[1])
-    assert theirs.search(qs[0], retrieval_unit=unit, top_k=2, truecase=False) == ours.search(qs[0], retrieval_unit=unit, top_k=2, truecase=False)
+    selection) run UNMODIFIED over this repo's MIPS / query2vec (search_setup) returned what the golden file records; densephrases_b200's
+    DensePhrases.search returns exactly that."""
+    from densephrases import DensePhrases
+    want = reference_golden("search")[unit]
+    ours = DensePhrases.__new__(DensePhrases)
+    ours.query2vec, ours.mips, ours.args = search_setup(oracle)
+    ours.truecase = None
+    got = search_outputs(ours, unit)
+    assert len(got["answers"]) == 3 and all(len(x) <= 3 for x in got["answers"])
+    assert got["answers"] == want["answers"] and got["single"] == want["single"]
+    no_score = lambda meta: [[{k: v for k, v in r.items() if k != "score"} for r in rets] for rets in meta]
+    assert no_score(got["meta"]) == no_score(want["meta"])
+    # the scores pass through the host BLAS (OPQ matrix, query vectors), whose fp32 summation order depends on the CPU it runs on
+    assert [r["score"] for rets in got["meta"] for r in rets] == pytest.approx([r["score"] for rets in want["meta"] for r in rets], rel=1e-5)
 
 
 def test_open_utils_and_single_utils_helpers_equal_unmodified_reference(tmp_path):
-    """`load_qa_pairs` (open_utils.py:103-163) and `backward_compat` (single_utils.py:36-56), the reference's code loaded by path
-    (its imports of squad_utils / embed_utils -- not on this path -- stubbed), against the facade's versions on awkward inputs."""
-    if not os.path.exists("/root/reference/densephrases/utils/open_utils.py"):
-        pytest.skip("reference tree not present (GPU box)")
-    import importlib.util
-    import sys
-    import types
+    """`load_qa_pairs` (open_utils.py:103-163) and `backward_compat` (single_utils.py:36-56): the reference's code (its imports of
+    squad_utils / embed_utils -- not on this path -- stubbed) on awkward inputs returned what the golden file records; the facade's
+    versions return the same."""
     from densephrases.utils import open_utils as mine_open, single_utils as mine_single
-    stubs = {"densephrases.utils.squad_utils": ("get_question_dataloader", "TrueCaser"), "densephrases.utils.embed_utils": ("get_question_results",)}
-    for name, attrs in stubs.items():
-        m = types.ModuleType(name)
-        for a in attrs:
-            setattr(m, a, object)
-        sys.modules[name] = m
-    try:
-        mods = {}
-        for short in ("single_utils", "open_utils"):
-            spec = importlib.util.spec_from_file_location(f"ref_{short}", f"/root/reference/densephrases/utils/{short}.py")
-            mods[short] = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(mods[short])
-    finally:
-        for name in stubs:
-            del sys.modules[name]
-    data = {"data": [{"id": "a1", "question": "Which river?", "answers": ["Seine"]},
-                     {"id": "a2", "origin": "nq.dev.x", "question": "who signed it", "answers": ["Louis", "Anne"], "titles": ["T1", "T2"]},
-                     {"id": "a3", "question": "skipped", "answers": []},
-                     {"id": "a4", "question": "x" * 400 + " [START_ENT] Paris [END_ENT] " + "y" * 400 + "?", "answers": ["Paris"]},
-                     {"id": "a5", "question": "ALL CAPS?", "answers": ["x"]}]}
+    g = reference_golden("qa_pairs")
     p = tmp_path / "qa.json"
-    json.dump(data, open(p, "w"))
-
-    class Args:
-        do_lower_case, draft, truecase, truecase_path = False, False, False, ""
-
-    for lower, q_idx in [(False, None), (True, None), (False, 1), (False, 3)]:
-        Args.do_lower_case = lower
-        want = mods["open_utils"].load_qa_pairs(str(p), Args, q_idx=q_idx)
-        got = mine_open.load_qa_pairs(str(p), Args, q_idx=q_idx)
-        assert [list(x) for x in got] == [list(x) for x in want]
-    sd = {"bert_q_start.embeddings.w": 1, "bert_q_end.x": 2, "bert_start.y": 3, "cross_encoder.z": 4, "bert_qd.q": 5, "qa_outputs.w": 6,
-          "query_start_encoder.k": 7, "linear.weight": 8}
-    assert mine_single.backward_compat(sd) == mods["single_utils"].backward_compat(sd)
+    json.dump(QA_PAIRS_DATA, open(p, "w"))
+    for (lower, q_idx), want in zip(QA_PAIRS_CONFIGS, g["load_qa_pairs"], strict=True):
+        QaPairsArgs.do_lower_case = lower
+        got = mine_open.load_qa_pairs(str(p), QaPairsArgs, q_idx=q_idx)
+        assert jsonable([list(x) for x in got]) == want
+    assert jsonable(mine_single.backward_compat(dict(BACKWARD_COMPAT_SD))) == g["backward_compat"]
 
 
 def test_option_flags_and_defaults_equal_reference_parser():
     """Every flag of the four option groups eval_phrase_retrieval.py / model.py add (options.py: model, index, retrieval, data)
-    exists here with the same default; nothing is renamed."""
-    if not os.path.exists("/root/reference/densephrases/options.py"):
-        pytest.skip("reference tree not present (GPU box)")
-    import importlib.util
+    exists here with the same default; nothing is renamed.  The reference parser's values are recorded in the golden file."""
     from densephrases import Options
-    spec = importlib.util.spec_from_file_location("ref_options", "/root/reference/densephrases/options.py")
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    theirs, ours = mod.Options(), Options()
-    for group in ("add_model_options", "add_index_options", "add_retrieval_options", "add_data_options"):
-        getattr(theirs, group)()
+    g = reference_golden("options")
+    ours = Options()
+    for group in OPTION_GROUPS:
         getattr(ours, group)()
-    want, got = vars(theirs.parser.parse_args([])), vars(ours.parse([]))
+    want, got = g["defaults"], jsonable(vars(ours.parse([])))
     assert not [k for k in want if k not in got]
     assert {k: got[k] for k in want} == want
-    argv = ["--cuda", "--top_k", "40", "--nprobe", "64", "--index_name", "start/1048576_flat_OPQ96", "--eval_batch_size", "32", "--agg_strat", "opt2"]
-    got2 = vars(ours.parse(argv))
-    assert {k: got2[k] for k in want} == vars(theirs.parser.parse_args(argv))
+    got2 = jsonable(vars(ours.parse(OPTION_ARGV)))
+    assert {k: got2[k] for k in g["argv"]} == g["argv"]
 
 
 def test_synthetic_dump_spec_objects(tmp_path):
@@ -402,40 +413,16 @@ def test_load_qa_pairs_truecases_lower_case_questions(tmp_path, monkeypatch, cap
 
 
 def test_truecaser_differential_against_the_reference_class():
-    """In the build container the reference tree is present: run the UNMODIFIED `TrueCaser` source (cut out of squad_utils.py with
-    `ast`, like tests/golden/make_truecase_golden.py) next to ours on fresh random sentences -- every output string and every score
-    must be equal.  (On the GPU box the tree does not exist; the committed golden file covers that case.)"""
-    ref_file = "/root/reference/densephrases/utils/squad_utils.py"
-    if not os.path.exists(ref_file):
-        pytest.skip("reference tree not present (GPU box)")
-    import ast, math, pickle, random, string, tempfile
-    from collections import defaultdict
+    """The UNMODIFIED `TrueCaser` source (cut out of squad_utils.py with `ast`, like tests/golden/make_truecase_golden.py) was run on
+    random sentences and score queries (truecase_differential_inputs); ours gives every output string and every score it recorded."""
+    import pickle
     from densephrases_b200.truecase import TrueCaser
-
-    def cut(path, name):
-        src = open(path).read()
-        node = next(n for n in ast.parse(src).body if getattr(n, "name", None) == name)
-        return ast.get_source_segment(src, node)
-    ns = {"os": os, "pickle": pickle, "math": math, "string": string}
-    exec(cut("/root/reference/densephrases/utils/data_utils.py", "whitespace_tokenize"), ns)
-    exec(cut(ref_file, "TrueCaser"), ns)
-    here = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "truecase.dist")
-    tables = pickle.load(open(here, "rb"))
-    with tempfile.NamedTemporaryFile(suffix=".dist", delete=False) as f:      # the reference indexes its count tables with []
-        pickle.dump({k: (defaultdict(int, v) if k != "word_casing_lookup" else v) for k, v in tables.items()}, f)
-    try:
-        ref, ours = ns["TrueCaser"](f.name), TrueCaser(here)
-        rng = random.Random(12345)
-        vocab = list(tables["word_casing_lookup"]) + ["zzz", "o'brien", "42", "?", ",", "'s", "x-ray", "Ünïcode", "a.b"]
-        for _ in range(400):
-            s = " ".join(rng.choice(vocab) for _ in range(rng.randint(0, 12)))
-            s = rng.choice([s, s.upper(), s.title(), "  " + s + " "])
-            for oov in ("title", "lower", "as-is"):
-                assert ours.get_true_case(s, oov) == ref.get_true_case(s, oov), (s, oov)
-        multi = [w for w, c in tables["word_casing_lookup"].items() if len(c) > 1]
-        for _ in range(300):
-            tok = rng.choice(tables["word_casing_lookup"][rng.choice(multi)])
-            prev, nxt = rng.choice([None] + vocab), rng.choice([None] + vocab)
-            assert ours.get_score(prev, tok, nxt) == ref.get_score(prev, tok, nxt)
-    finally:
-        os.unlink(f.name)
+    here = os.path.join(GOLD, "truecase.dist")
+    g = reference_golden("truecase_differential")
+    cases, scores = truecase_differential_inputs(pickle.load(open(here, "rb")))
+    ours = TrueCaser(here)
+    assert len(cases) == len(g["cases"]) and len(scores) == len(g["scores"])
+    for (s, oov), want in zip(cases, g["cases"]):
+        assert ours.get_true_case(s, oov) == want, (s, oov)
+    for (prev, tok, nxt), want in zip(scores, g["scores"]):
+        assert ours.get_score(prev, tok, nxt) == want, (prev, tok, nxt)

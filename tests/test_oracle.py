@@ -1,15 +1,10 @@
 """CPU tests of the oracle itself (the reference holds no golden vectors for this path, SURVEY.md 8c):
 C restatement == numpy restatement bit-for-bit, both == exhaustive fp64 scoring, heap/tie/padding semantics,
 and the committed golden fixtures (tests/golden/make_golden.py) still reproduce."""
-import json
-import os
-
 import numpy as np
 import pytest
 
-from tests.helpers import near_queries, opq_matrix, uniform_lens
-
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
+from tests.helpers import load_ivfpq_small, near_queries, opq_matrix, uniform_lens
 
 
 def small_index(oracle, nlist=16, seed=11, lens=None, explicit=False):
@@ -110,8 +105,7 @@ def test_resident_lists_view_is_equivalent(oracle):
 
 
 def test_golden_fixture_reproduces(oracle):
-    g = np.load(os.path.join(GOLD, "ivfpq_small.npz"))
-    meta = json.load(open(os.path.join(GOLD, "ivfpq_small.json")))
+    g, meta = load_ivfpq_small(oracle)
     ix = oracle.RefIndex(g["A"], g["pq"], g["list_len"], centroids=g["centroids"], codes=g["codes"], ids=g["ids"])
     D, I, key = ix.search(g["x"], meta["k"], meta["nprobe"], return_key=True)
     assert np.array_equal(D.view(np.int32), g["D"].view(np.int32)) and np.array_equal(I, g["I"]) and np.array_equal(key, g["key"])

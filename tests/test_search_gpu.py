@@ -3,7 +3,7 @@ Integer/index outputs bit-exact; fp32 scores bit-identical (stricter than the 1e
 import numpy as np
 import pytest
 
-from tests.helpers import assert_topk_equal, near_queries, opq_matrix, uniform_lens
+from tests.helpers import assert_topk_equal, load_ivfpq_small, near_queries, opq_matrix, uniform_lens
 
 pytestmark = pytest.mark.gpu
 SEED = 1234
@@ -133,13 +133,9 @@ def test_device_tensor_api_and_fast_equals_exact(oracle):
     assert_topk_equal(D0.cpu().numpy(), I0.cpu().numpy(), Dr, Ir)
 
 
-def test_golden_fixture_on_gpu():
-    import json
-    import os
+def test_golden_fixture_on_gpu(oracle):
     from densephrases_b200 import IvfPqIndex
-    gd = os.path.join(os.path.dirname(__file__), "golden")
-    g = np.load(os.path.join(gd, "ivfpq_small.npz"))
-    meta = json.load(open(os.path.join(gd, "ivfpq_small.json")))
+    g, meta = load_ivfpq_small(oracle)
     for mode in (3, 2, 1):
         ix = IvfPqIndex(len(g["list_len"]))
         ix.set_opq(g["A"]); ix.set_pq(g["pq"]); ix.set_centroids(g["centroids"]); ix.set_lists(g["list_len"], g["codes"], g["ids"])
