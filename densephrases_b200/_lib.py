@@ -65,6 +65,8 @@ _SIGS = {
     "dph_encoder_tower_floats": (_i64, [_vp]),
     "dph_encoder_load_tower": (_i32, [_vp, _i32, _vp, _i32]),
     "dph_encoder_embed_query": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _i32]),
+    "dph_encoder_load_filter": (_i32, [_vp, _vp, _vp, _i32]),
+    "dph_encoder_embed_phrase": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _f32, _f32, _i32]),
     "dph_sgemm_nt_seq": (_i32, [_vp, _i64, _vp, _i64, _i64, _vp, _vp]),
     "dph_gemm_tf32_nt": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i32, _i32, _vp]),
     "dph_encoder_set_precision": (_i32, [_vp, _i32]),

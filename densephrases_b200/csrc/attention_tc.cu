@@ -425,25 +425,27 @@ __global__ void __launch_bounds__(128, 2) attention_tc_bx_kernel(const __grid_co
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(256) : "memory");
 }
 
-// qkv[t]: [T, 2304] fp32 (Q | K | V, heads contiguous inside each), ctx[t]: [T, 768]; mask int64 [B, S]; S <= 64, 12 heads.
+// qkv[t]: [T, 2304] fp32 (Q | K | V, heads contiguous inside each), ctx[t]: [T, 768]; mask int64 [B, S]; S <= 64, 12 heads;
+// towers t < ntw (blockIdx.z).
 int dph_launch_attention_tc(const float* const qkv[2], float* const ctx[2], const long long* mask, int B, int S, long long T, cudaStream_t st, int split,
-                            unsigned short* const* ctx_hi, unsigned short* const* ctx_lo) {
+                            unsigned short* const* ctx_hi, unsigned short* const* ctx_lo, int ntw) {
     DPH_CHECK(S >= 1 && S <= 64 && B >= 1 && T >= (long long)B * S, "attention_tc: S must be 1..64");
+    DPH_CHECK(ntw == 1 || ntw == 2, "attention_tc: one or two towers");
     static DphPerDeviceOnce once;
     if (once.first()) {
         DPH_CUDA(cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AT_SMEM_BYTES));
         DPH_CUDA(cudaFuncSetAttribute(attention_tc_bx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATB_SMEM_BYTES));
     }
-    AttnTcMaps maps;
-    AttnTcArgs a;
-    for (int t = 0; t < 2; t++) {
+    AttnTcMaps maps = {};
+    AttnTcArgs a = {};
+    for (int t = 0; t < ntw; t++) {
         DPH_TRY(dph_make_map_f32(&maps.qkv[t], qkv[t], T, 3 * AT_H, 3 * AT_H, 64));
         a.qkv[t] = qkv[t]; a.ctx[t] = ctx[t];
         a.ctx_hi[t] = ctx_hi ? ctx_hi[t] : nullptr; a.ctx_lo[t] = ctx_lo ? ctx_lo[t] : nullptr;
     }
     a.mask = mask; a.S = S;
-    if (split) attention_tc_bx_kernel<<<dim3(6, (unsigned)B, 2), 128, ATB_SMEM_BYTES, st>>>(maps, a);
-    else attention_tc_kernel<<<dim3(6, (unsigned)B, 2), 128, AT_SMEM_BYTES, st>>>(maps, a);
+    if (split) attention_tc_bx_kernel<<<dim3(6, (unsigned)B, (unsigned)ntw), 128, ATB_SMEM_BYTES, st>>>(maps, a);
+    else attention_tc_kernel<<<dim3(6, (unsigned)B, (unsigned)ntw), 128, AT_SMEM_BYTES, st>>>(maps, a);
     DPH_CUDA(cudaGetLastError());
     return 0;
 }

@@ -18,7 +18,7 @@ from collections import Counter
 import numpy as np
 import torch
 
-from .encoder import BertGeometry, Encoder, random_state_dict
+from .encoder import BertGeometry, Encoder, random_filter_state_dict, random_state_dict
 from .mips import MIPS
 from .options import Options
 from .tokenization import WordPieceTokenizer
@@ -112,9 +112,9 @@ def load_encoder(device, args, phrase_only=False):
     """-> (model, tokenizer, config) from `args.load_dir/pytorch_model.bin` + a WordPiece `vocab.txt` (single_utils.py:59-118).
     A missing checkpoint or vocabulary raises FileNotFoundError like the reference does; seeded random weights and the
     synthetic character-level vocabulary are used only when the caller opts in with `args.allow_random_init = True` or the
-    environment variable DPH_ALLOW_RANDOM_INIT=1 (tests and benchmarks: no checkpoint is reachable offline)."""
-    if phrase_only:
-        raise NotImplementedError('the phrase tower is only used offline (generate_phrase_vecs.py); out of scope')
+    environment variable DPH_ALLOW_RANDOM_INIT=1 (tests and benchmarks: no checkpoint is reachable offline).
+    phrase_only=True (generate_phrase_vecs.py): the phrase tower and the filter head only, like the reference's
+    `del model.query_start_encoder` / `del model.query_end_encoder` (single_utils.py:106-114)."""
     load_dir = getattr(args, 'load_dir', '') or ''
     allow_random = bool(getattr(args, 'allow_random_init', False)) or os.environ.get('DPH_ALLOW_RANDOM_INIT', '') == '1'
     config = BertGeometry()
@@ -138,12 +138,17 @@ def load_encoder(device, args, phrase_only=False):
         sd = backward_compat(torch.load(ckpt, map_location='cpu'))
         logger.info(f'DensePhrases encoder loaded from {load_dir}')
     elif allow_random:
-        sd = random_state_dict(config, getattr(args, 'seed', 42))
-        logger.warning('no checkpoint found: query encoder initialised with seeded random weights (allow_random_init)')
+        seed = getattr(args, 'seed', 42)
+        if phrase_only:
+            sd = random_state_dict(config, seed, prefixes=('phrase_encoder',))
+            sd.update(random_filter_state_dict(config, seed))
+        else:
+            sd = random_state_dict(config, seed)
+        logger.warning('no checkpoint found: encoder initialised with seeded random weights (allow_random_init)')
     else:
         raise FileNotFoundError(f'{ckpt} not found (hub ids are not resolvable offline); pass allow_random_init=True for seeded random weights')
     dev_index = torch.cuda.current_device() if str(device).startswith('cuda') else 0
-    model = Encoder(config, tokenizer=tokenizer, state_dict=sd, device=dev_index)
+    model = Encoder(config, tokenizer=tokenizer, state_dict=sd, device=dev_index, towers='phrase' if phrase_only else 'query')
     return model, tokenizer, config
 
 

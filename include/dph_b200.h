@@ -141,31 +141,45 @@ int dph_index_reconstruct_batch(dph_index* ix, const int64_t* ids, int64_t m, fl
 int dph_index_window_scores(dph_index* ix, const float* q /*[m,d]*/, const int64_t* first_id /*[m]*/, int64_t m, int L,
                             float* out_scores, int mem);
 
-/* ---- query encoder (replaces Encoder.forward(return_query=True) -> embed_query, densephrases/encoder.py:146-152,101-118) ----
- * Two BERT-base towers (12 layers, 768 hidden, 12 heads, 3072 FFN; SpanBERT-base-cased geometry, options.py:23) on the same
- * tokens.  tower 0 = query_start_encoder.*, tower 1 = query_end_encoder.* (encoder.py:51-52).  Weight blob layout: encoder.cu. */
+/* ---- encoder (replaces Encoder.forward(return_query=True) -> embed_query, densephrases/encoder.py:146-152,101-118, and
+ * Encoder.forward(input_ids=..., return_phrase=True) -> embed_phrase + filter_linear, encoder.py:92-99,130-144) ----
+ * BERT-base towers (12 layers, 768 hidden, 12 heads, 3072 FFN; SpanBERT-base-cased geometry, options.py:23).  tower 0 =
+ * query_start_encoder.*, tower 1 = query_end_encoder.*, tower 2 = phrase_encoder.* (encoder.py:50-52); each is allocated only when
+ * loaded.  Weight blob layout: encoder.cu. */
 typedef struct dph_encoder dph_encoder;
 int dph_encoder_create(dph_encoder** out, int device, int vocab_size, int max_position_embeddings, int type_vocab_size);
 void dph_encoder_free(dph_encoder* e);
 int dph_encoder_set_stream(dph_encoder* e, void* cuda_stream);
 int64_t dph_encoder_tower_floats(const dph_encoder* e);
 int dph_encoder_load_tower(dph_encoder* e, int tower, const float* blob, int mem);
+/* filter_linear (encoder.py:32): W fp32 [2,768] (row 0: start logit, row 1: end logit), b fp32 [2]. */
+int dph_encoder_load_filter(dph_encoder* e, const float* W, const float* b, int mem);
 /* 0 (default): GEMMs as one TF32 MMA per product -- what torch 1.9 (the reference's pin) does for fp32 matmuls on Ampere+;
  * 1: 3xTF32 split GEMMs, fp32-accurate (matches the reference's CPU/fp32 path to ~1e-5);
  * 2: bf16x3 split GEMMs (operands as (hi, lo) bf16 planes, three kind::f16 MMAs per product, ~2^-17 relative): meets the 1e-3
  *    tolerance on the query vectors at the speed of mode 0. */
 int dph_encoder_set_precision(dph_encoder* e, int precise);
-/* 1 (default): self-attention of sequences with S <= 64 on the tensor cores -- TF32 operands in precision mode 0, bf16 (hi, lo) planes with three
- * MMAs per contraction (fp32-accurate) in modes 1 and 2; fp32 accumulation and softmax.  0: always the fp32 SIMT attention kernels. */
+/* 1 (default): self-attention of sequences with S <= 64 (and, in the phrase forward, 64 < S <= 512) on the tensor cores -- TF32
+ * operands in precision mode 0, bf16 (hi, lo) planes with three MMAs per contraction (fp32-accurate) in modes 1 and 2; fp32
+ * accumulation and softmax.  0: always the fp32 SIMT attention kernels (S <= 384). */
 int dph_encoder_set_attention(dph_encoder* e, int tensor_core);
 /* One BERT-base self-attention (12 heads x 64; HF BertSelfAttention as used by encoder.py:101-118) on device buffers:
- * qkv fp32 [B*S, 2304] = (Q | K | V), mask int64 [B,S] -> ctx fp32 [B*S, 768].  tensor_core: 0 SIMT fp32, 1 tcgen05 TF32,
- * 2 tcgen05 on bf16 (hi, lo) operand planes, three MMAs per contraction (fp32-accurate); 1 and 2 need S <= 64. */
+ * qkv fp32 [B*S, 2304] = (Q | K | V), mask int64 [B,S] -> ctx fp32 [B*S, 768].  tensor_core: 0 SIMT fp32 (S <= 384),
+ * 1 tcgen05 TF32, 2 tcgen05 on bf16 (hi, lo) operand planes, three MMAs per contraction (fp32-accurate); 1 and 2: S <= 512 (S > 64
+ * runs the long-sequence kernel with an online softmax over key tiles). */
 int dph_attention_bert(const float* qkv, const int64_t* attention_mask, int B, int S, float* ctx, int tensor_core, void* cuda_stream);
 /* input_ids / attention_mask / token_type_ids int64 [B,S] (S <= 384); start_out / end_out fp32 [B,768] = hidden state at
  * position 0 of each tower (the reference returns them as [B,1,768]). */
 int dph_encoder_embed_query(dph_encoder* e, const int64_t* input_ids, const int64_t* attention_mask, const int64_t* token_type_ids,
                             int B, int S, float* start_out, float* end_out, int mem);
+/* Phrase tower over every token: input_ids / attention_mask / token_type_ids int64 [B,S], 1 <= S <= min(512, max_position_embeddings).
+ * out fp32 [B,S,768] (nullable) = the last hidden state (start == end in the reference); filter_start / filter_end fp32 [B,S] =
+ * filter_linear logits; out_q int8 [B,S,768] (nullable) = float_to_int8(out, dense_offset, dense_scale) (embed_utils.py:141-145:
+ * fp32 (x - offset) * scale, clamped to [-128, 127], rounded half to even).  Needs tower 2 and the filter head.  Buffers and the
+ * out-of-range id flag follow dph_encoder_embed_query. */
+int dph_encoder_embed_phrase(dph_encoder* e, const int64_t* input_ids, const int64_t* attention_mask, const int64_t* token_type_ids,
+                             int B, int S, float* out, float* filter_start, float* filter_end, int8_t* out_q, float dense_offset,
+                             float dense_scale, int mem);
 
 /* ---- exact sequential-k fp32 GEMM (the inner-product definition shared with the oracle): out [n,m] = X [n,K] . W [m,K]^T,
  * acc = fmaf(x[t], w[t], acc) for t ascending; device pointers; K % 32 == 0.  Used for the OPQ rotation and the coarse quantizer. */
